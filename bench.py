@@ -19,6 +19,12 @@ Inputs (530 MB per GPU) exceed the 126 MB L2, so no L2 flush is needed between i
               NOT HBM bound (2.3 B/window): the fraction is reported as it is.
   cpu_baseline / --impl reference : the CPU restatement of the reference (oracle/, kind "port" -- the reference is Go
               and no Go toolchain exists here) on the host cores, frame-parallel, bounded sample.
+
+--dump-outputs DIR writes what the last timed step returned to its caller (rank 0's frame-ordered result) as float32 .npy
+files, so that two builds can be compared output for output: the frames are seeded, identical from run to run.
+  counts.npy       [frames]             detections found per frame (may exceed the 1024 slots of a frame)
+  detections.npy   [frames, 1024, 4]    (row, col, scale, score) per slot, zero past the frame's count
+  frame_index.npy  [frames]             which frames of the step these are (a seeded sample when all would exceed 64 MB)
 """
 from __future__ import annotations
 
@@ -133,6 +139,25 @@ def cpu_sample_frames(nthreads: int, requested: int) -> int:
     return requested or max(16, min(512, 4 * nthreads))
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(dirname: str, dets: np.ndarray, counts: np.ndarray):
+    """dets: [frames, cap, 4] int32 (row, col, scale, float32 bits of the score), counts: [frames] int32; see --dump-outputs."""
+    nf, cap = dets.shape[:2]
+    keep = max(1, DUMP_LIMIT_BYTES // (cap * 16 + 8))
+    idx = np.arange(nf) if nf <= keep else np.sort(np.random.default_rng(0).choice(nf, keep, replace=False))
+    d, c = dets[idx], counts[idx]
+    out = np.empty(d.shape, dtype=np.float32)
+    out[..., :3] = d[..., :3]
+    out[..., 3] = d.view(np.float32)[..., 3]
+    out[np.arange(cap)[None, :] >= np.minimum(c, cap)[:, None]] = 0   # slots past the count hold nothing a caller may read
+    os.makedirs(dirname, exist_ok=True)
+    np.save(os.path.join(dirname, "detections.npy"), out)
+    np.save(os.path.join(dirname, "counts.npy"), c.astype(np.float32))
+    np.save(os.path.join(dirname, "frame_index.npy"), idx.astype(np.float32))
+
+
 def _claim_stdout():
     """The contract is ONE JSON line on stdout: everything else any library writes to fd 1 (NCCL prints its version
     banner there at WARN level, torchrun children inherit the fd) is sent to stderr; the line itself goes to the saved fd."""
@@ -159,7 +184,12 @@ def main():
     ap.add_argument("--no-extra", action="store_true", help="skip the configs[3] / configs[4] blocks (developer runs)")
     ap.add_argument("--pipeline-frames", type=int, default=64, help="frames per GPU per step of the configs[4] pipeline block")
     ap.add_argument("--opts", default="", help="developer sweeps: library options as name=value,... (default: none)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's detections to DIR/*.npy (see the module doc)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the GPU path's outputs; it does not apply to --impl reference")
     out_fd = _claim_stdout()
 
     rank = int(os.environ.get("RANK", "0"))
@@ -225,10 +255,12 @@ def main():
     st = stream.cuda_stream
 
     def step_device():
+        """Returns what the step hands its caller: this rank's (dets, counts), or for N>1 the gathered lists on rank 0."""
         clf.run_cascade_batch_device(d_frames.data_ptr(), nf, ROWS * COLS, ROWS, COLS, COLS, *PARAMS, 0.0,
                                      d_out.data_ptr(), cap, d_cnt.data_ptr(), st)
         if world > 1:
-            pdist.gather_detections(d_out, d_cnt, dst=0)
+            return pdist.gather_detections(d_out, d_cnt, dst=0)
+        return [d_out], [d_cnt]
 
     def barrier():
         if world > 1:
@@ -256,11 +288,15 @@ def main():
     barrier()
     e0.record(stream)
     for _ in range(args.steps):
-        step_device()
+        last = step_device()
     e1.record(stream)
     barrier()
     ms_total = max_over_ranks(e0.elapsed_time(e1))
     launches = pigo_b200.launch_count() - launches0
+    dumped = None
+    if args.dump_outputs and rank == 0:   # copied now: the passes below overwrite d_out / d_cnt
+        dets_last, cnt_last = pdist.merge_gathered(*last, nf * world)
+        dumped = (dets_last.cpu().numpy(), cnt_last.cpu().numpy())
     for _ in range(args.steps):   # keep the GPU under the same load while the sampler collects a few more points
         step_device()
     torch.cuda.synchronize()
@@ -554,6 +590,8 @@ def main():
                         "single_thread_value": v1, "host": host_info(), "note": "C -O2 restatement of core/pigo.go (oracle/); the Go "
                         "reference cannot be built in this image (no Go toolchain)"}
 
+    if dumped is not None:
+        dump_outputs(args.dump_outputs, *dumped)
     if rank == 0:
         _emit(out_fd, {
             "metric": "candidate windows/s on 1080p frames", "value": value, "unit": "windows/s", "n_gpus": world,
